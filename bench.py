@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle's C restatement on the host cores
     python bench.py --workload wcci --gpus N ...             # BASELINE.json configs[4]: 118 substations, batch 8192 in total
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's results as DIR/<name>.npy (float32)
 
 Workload `case14` (default; BASELINE.json configs[1], the configuration the metric is quoted on): l2rpn_case14_sandbox, AC
 Newton-Raphson, batch 4096 per GPU (weak scaling), DoNothing rollout over the bundled chronics (instance i -> scenario i mod 3,
@@ -247,6 +248,7 @@ class CpuArm:
         out, status, iters, _ = self.orc.run(self.topo, self.inj)
         dt = time.perf_counter() - t
         assert (status == 0).all()
+        self.last = (out, status, iters)
         return dt
 
     def sample(self, min_steps, min_seconds, warmup=2):
@@ -279,7 +281,11 @@ def run_reference(args):
     gm, chron = load_workload(args.workload)
     batch = args.batch or (w["batch_per_gpu"] or w["total_batch"])
     arm = CpuArm(gm, chron, batch)
-    ts = arm.sample(args.steps, max(2.0, args.cpu_min_seconds), warmup=max(args.warmup, 1))
+    ts = arm.sample(args.steps, args.cpu_min_seconds, warmup=max(args.warmup, 1))
+    if args.dump_outputs:
+        from grid2op_b200.engine import OutputView
+        out, status, iters = arm.last
+        dump_outputs(args.dump_outputs, gm, out, status, iters, OutputView(gm, out).a_or / gm.thermal_limit_a[None, :])
     rates = batch / ts
     value = float(np.median(rates))
     line = {
@@ -290,7 +296,7 @@ def run_reference(args):
         "config": {"workload": f"{w['env']} AC Newton-Raphson, batch {batch} envs per GPU, DoNothing rollout", "batch_per_step": batch,
                    "arm": "host CPU: one batch of that size per step, all host threads the cgroup grants",
                    "requested_steps": args.steps,
-                   "note": "value = median over the steps of batch / step time; the arm runs at least 2 s whatever --steps says"},
+                   "note": "value = median over the steps of batch / step time; --cpu-min-seconds > 0 adds steps until the arm has run that long"},
         "spread": {"min": float(rates.min()), "median": value, "max": float(rates.max()), "unit": UNIT, "n": int(len(ts))},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": arm.nthreads, "kind": "port", "sample": arm.describe(ts),
                          "host": arm.info},
@@ -298,6 +304,32 @@ def run_reference(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, gm, out, status, iters, rho):
+    """``--dump-outputs``: what the timed path returned for its last step as ``<dirname>/<name>.npy`` (float32): ``rho``,
+    every field of the result record (engine.OutputView) the grid has elements for, the solver ``status`` and Newton
+    ``iterations`` per instance.  Above 64 MB in all, a fixed seeded sample of instances is written, their indices in
+    ``instance.npy``."""
+    from grid2op_b200.engine import OutputView
+    idx = np.arange(len(status))
+    row_bytes = 4 * (gm.n_out + gm.n_line + 2)
+    if len(idx) * row_bytes > DUMP_LIMIT_BYTES:
+        n = (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 4)
+        idx = np.sort(np.random.default_rng(0).choice(len(idx), n, replace=False))
+    view = OutputView(gm, out[idx])
+    arrays = {"rho": rho[idx], "status": status[idx], "iterations": iters[idx]}
+    arrays.update((name, getattr(view, name)) for name in OutputView.FIELDS)
+    if len(idx) < len(status):
+        arrays["instance"] = idx
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size == 0:                 # no element of that kind (e.g. no storage unit on the grid)
+            continue
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -462,6 +494,8 @@ def run_ours(args):
 
     # ---- self-checks of what was just timed -----------------------------------------------------------------------------
     out_h, status_h, iters_h, rho_h = eng.series_fetch()      # rho_h is read back from wherever the kernel stored it (rank 0's HBM)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gm, out_h, status_h, iters_h, rho_h)
     from grid2op_b200.engine import OutputView
     a_or = OutputView(gm, out_h).a_or
     collected_ok = bool(np.allclose(rho_h, a_or / gm.thermal_limit_a[None, :].astype(np.float32), rtol=1e-6, atol=0, equal_nan=True))
@@ -632,13 +666,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="instances per GPU (default: the workload's)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="length of the in-run cpu_baseline sample (N=1)")
-    ap.add_argument("--cpu-min-seconds", type=float, default=4.0, help="--impl reference: run at least this long whatever --steps")
+    ap.add_argument("--cpu-min-seconds", type=float, default=0.0, help="--impl reference: time more than --steps steps until this long")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-redo", action="store_true", help="measurement only: planned kernel without its pivoting safety net")
     ap.add_argument("--gather-every", type=int, default=64, help="N>1: steps per arrival signal / gather")
     ap.add_argument("--collect", default="nccl", choices=["p2p", "nccl"], help="N>1: how rho reaches rank 0")
     ap.add_argument("--policy", type=int, default=0, choices=[0, 1, 2],
                     help="kernel policy (include/b200pf.h): 0 auto = planned kernel, 1 pivoting kernels only, 2 planned always")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (float32, at most 64 MB; rank 0's instances)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

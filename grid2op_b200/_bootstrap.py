@@ -1,7 +1,8 @@
 """Locate an importable ``grid2op`` (the host framework we plug into; NOT re-implemented here).
 
-Search order: an already importable ``grid2op`` -> ``$GRID2OP_B200_REF`` -> ``<repo>/baseline/_ref``
-(the unmodified reference installed with ``pip install --target``; git-ignored).  Nothing else is searched: a checkout
+Search order: an already importable ``grid2op`` -> ``$GRID2OP_B200_REF`` -> ``<repo>/oracle/_ref`` (the unmodified
+reference installed by ``build()``, oracle/reference.py; git-ignored) -> ``<repo>/baseline/_ref`` (the same installed with
+``pip install --target``; git-ignored).  Nothing else is searched: a checkout
 elsewhere is named through the environment variable (tests/conftest.py does that for the build container).
 
 grid2op imports ``pandapower`` at package-import time (reference:
@@ -22,6 +23,7 @@ import types
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _CANDIDATES = [
     os.environ.get("GRID2OP_B200_REF", ""),
+    os.path.join(_REPO, "oracle", "_ref"),
     os.path.join(_REPO, "baseline", "_ref"),
 ]
 

@@ -1,5 +1,5 @@
-"""Build recipe of the C restatement (oracle/pf_oracle.c -> oracle/libpf_oracle.so).  The reference is
-pure Python (no C/C++ sources under /root/reference), so there is no oracle/_ref to compile."""
+"""Build recipe of the C restatement (oracle/pf_oracle.c -> oracle/libpf_oracle.so).  The reference is pure Python: its
+install into oracle/_ref is oracle/reference.py."""
 import os
 import sys
 

@@ -6,11 +6,8 @@ import pytest
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
-# In the build container the full reference tree (with its test-suites AND their data_test fixtures)
-# is mounted read-only: prefer it, so the extended reference suites with golden vectors run.  On the
-# GPU box only baseline/_ref (pip --target install of the unmodified reference) exists.
-if "GRID2OP_B200_REF" not in os.environ and os.path.isdir("/root/reference/grid2op/data_test"):
-    os.environ["GRID2OP_B200_REF"] = "/root/reference"
+# The reference (grid2op with its bundled data, test-suites and data_test fixtures) is found in $GRID2OP_B200_REF or in
+# oracle/_ref, where build() installs it (oracle/reference.py).
 
 
 def pytest_configure(config):
@@ -28,8 +25,8 @@ def grid2op_root():
     """Directory that contains the reference's ``grid2op`` package (for its bundled grid files)."""
     return _first_dir([
         os.path.join(os.environ.get("GRID2OP_B200_REF", ""), "grid2op") if os.environ.get("GRID2OP_B200_REF") else None,
+        os.path.join(REPO, "oracle", "_ref", "grid2op"),
         os.path.join(REPO, "baseline", "_ref", "grid2op"),
-        "/root/reference/grid2op",
     ])
 
 
@@ -42,7 +39,8 @@ def env_grid(name):
 
 
 def data_test_dir():
-    return _first_dir(["/root/reference/grid2op/data_test"])
+    root = grid2op_root()
+    return _first_dir([os.path.join(root, "data_test") if root else None])
 
 
 def have_cuda():

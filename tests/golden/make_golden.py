@@ -148,7 +148,34 @@ def env_chronics(env, out_name):
     return chron
 
 
+def simulate_forecast_fixture():
+    """-> simulate_forecast_case14.npz: rho of obs.simulate(do_nothing) of unmodified l2rpn_case14_sandbox environments
+    (the oracle's PandaPowerBackend restatement solving) behind reset and the first steps of the 3 bundled scenarios, with the
+    forecast rows the batched what-if reads for those steps (tests/test_simulate_forecast_gpu.py)"""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import grid2op_b200.backend as bk
+    from grid2op_b200.chronics import _open, list_scenarios, load_forecasts, load_scenarios
+    from oracle_engine import OracleEngine
+    from test_simulate_forecast_gpu import N_STEPS, obs_simulate_rho
+
+    class OracleBackend(bk.B200Backend):
+        def _make_engine(self, gm):
+            return OracleEngine(gm)
+
+    env = "l2rpn_case14_sandbox"
+    gm = GridModel(os.path.join(REF, env, "grid.json"))
+    folders = list_scenarios(os.path.join(REF, env, "chronics"))
+    stored = np.load(os.path.join(HERE, "case14_sandbox_chronics.npz"))["chron"]
+    assert np.array_equal(load_scenarios(os.path.join(REF, env, "chronics"), gm), stored)
+    fc = np.stack([load_forecasts(f, gm)[:N_STEPS] for f in folders])
+    has_pv = _open(os.path.join(folders[0], "prod_v_forecasted")) is not None
+    want, th = obs_simulate_rho(OracleBackend, len(folders))
+    np.savez_compressed(os.path.join(HERE, "simulate_forecast_case14.npz"), want=want, th=th, fc=fc, has_pv=has_pv)
+    return want.shape
+
+
 if __name__ == "__main__":
+    print("simulate forecast", simulate_forecast_fixture())
     print("data_test fixtures", data_test_fixtures())
     print("wcci chronics", env_chronics("l2rpn_wcci_2022_dev", "wcci_2022_dev_chronics.npz").shape)
     print("neurips track1 chronics", env_chronics("l2rpn_neurips_2020_track1", "neurips_2020_track1_chronics.npz").shape)

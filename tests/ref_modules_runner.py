@@ -21,7 +21,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE)); sys.path.insert(0, HERE)
 
 
-import conftest  # noqa: F401,E402  (points GRID2OP_B200_REF at the reference tree when it is there)
+import conftest  # noqa: F401,E402
 import grid2op_b200.backend as bk  # noqa: E402
 
 

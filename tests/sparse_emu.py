@@ -16,7 +16,10 @@ def build(force: bool = False) -> str:
     src = os.path.join(HERE, "sparse_emu.cpp")
     deps = [src] + [os.path.join(REPO, "grid2op_b200", "csrc", f) for f in ("b200pf_sparse.cuh", "b200pf_plan.hpp", "b200pf_block.cuh")]
     if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(p) for p in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-x", "c++", "-o", LIB, src, "-lm"])
+        # compiled under a private name and renamed into place: parallel test workers may build it at the same time
+        tmp = f"{LIB}.{os.getpid()}.tmp"
+        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-x", "c++", "-o", tmp, src, "-lm"])
+        os.replace(tmp, LIB)
     return LIB
 
 

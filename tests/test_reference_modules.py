@@ -12,7 +12,6 @@ import sys
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_TESTS = "/root/reference/grid2op/tests"
 
 # (backend-facing modules, each a few seconds at most)
 MODULES = [
@@ -51,7 +50,9 @@ def _run_modules():
 
 @pytest.fixture(scope="module")
 def results(request, tmp_path_factory):
-    if not os.path.isdir(REF_TESTS) or not os.path.isdir("/root/reference/grid2op/data_test"):
+    from conftest import grid2op_root
+    root = grid2op_root()
+    if root is None or not os.path.isdir(os.path.join(root, "tests")) or not os.path.isdir(os.path.join(root, "data_test")):
         pytest.skip("reference test tree (with its data_test fixtures) not available")
     uid = getattr(request.config, "workerinput", {}).get("testrunuid")
     if uid is None:                      # plain (serial) run
